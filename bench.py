@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - HSTU training sequences/sec (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE configs[1] - HSTU 4 blocks, d=128, h=4, seq_len=200, V=12,101 synthetic
@@ -57,7 +57,15 @@ def parse():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-eager", action="store_true")
     ap.add_argument("--skip-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss, parameters after the optimizer step) as "
+                         "DIR/<name>.npy in float32.  That step starts from the initial parameters and optimizer state and its batch "
+                         "and dropout seed follow from the arguments, so two runs or two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     c = CONFIGS[args.config]
     CFG.clear(); CFG.update(c["model"])
     args.batch = args.batch or c["batch"]
@@ -258,6 +266,11 @@ def run_ours(args, rank, world, local_rank):
     model = HSTU(**{**CFG, "max_seq_len": L}).to(dev).train()
     # plain loss.backward() every step: the head may accumulate straight into the flat gradient buffer (checked on the device)
     opt = FlatAdam(model, lr=1e-3, betas=(0.9, 0.98), unit_loss_grad=True, defer_weight_grads=os.environ.get("GRB_DEFER", "1") != "0")
+    # --dump-outputs: the gradient reductions use float atomics, so two runs agree only to rounding after one step, and Adam amplifies
+    # that difference with every further step.  The last timed step therefore starts again from the state before the first step (the
+    # only training state that is bit-identical from run to run): parameters, bf16 mirror, Adam moments and step count.  Restoring
+    # them adds one device copy to that step; without --dump-outputs the timed steps are unchanged.
+    initial = [t.clone() for t in (opt.flat, opt.mirror, opt.m, opt.v, opt.state)] if args.dump_outputs else None
 
     nb = 8
     host = [tuple(t.pin_memory() for t in synth_batch(B, L, V, 1000 * rank + i)) for i in range(nb)]
@@ -318,7 +331,11 @@ def run_ours(args, rank, world, local_rank):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(loader, sync_each):
+    def restore_initial():
+        for dst, src in zip((opt.flat, opt.mirror, opt.m, opt.v, opt.state), initial):
+            dst.copy_(src)
+
+    def timed(loader, sync_each, restart_last=False):
         for i in range(W):
             loader(i)
             run_step()
@@ -332,6 +349,8 @@ def run_ours(args, rank, world, local_rank):
         e0.record()
         marks[0].record()
         for i in range(K):
+            if restart_last and i == K - 1:
+                restore_initial()
             loader(W + i)
             run_step()
             if sync_each:
@@ -358,8 +377,10 @@ def run_ours(args, rank, world, local_rank):
         sampler.start()
     ms_dev, _, pct_dev = timed(load_resident, sync_each=False)
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e, wall_e2e, pct_e2e = timed(load_host, sync_each=True)
+    ms_e2e, wall_e2e, pct_e2e = timed(load_host, sync_each=True, restart_last=initial is not None)
     final_loss = float(loss_static.detach().float().item())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss_static, model)
 
     # ---- roofline of the HSTU block stack (fwd+bwd), device-timed inside a graph
     roof = None
@@ -404,6 +425,24 @@ def run_ours(args, rank, world, local_rank):
                          ms_per_step=ms_e2e / K, wall_ms_per_step=wall_e2e / K, ms_per_step_pct=pct_e2e),
                 gpu_launches=launches_per_step * K, clocks=clocks, roofline=roof, cpu_baseline=cpu, cuda_eager_baseline=eager)
     emit(line)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, loss, model):
+    """The caller of a training step receives the loss and the updated parameters: loss.npy and param.<name>.npy, float32.
+    Every parameter is written in full (36 MB at cfg3)."""
+    import numpy as np
+    arrays = {"loss": loss.detach()}
+    arrays.update({f"param.{n}": p.detach() for n, p in model.named_parameters()})
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # DRAM bytes (dram__bytes_read.sum + dram__bytes_write.sum) of the block stack's kernels for one fwd+bwd, from the committed ncu

@@ -15,6 +15,5 @@ vectors for this path (SURVEY.md section 4), so the oracle is pinned against
 outputs of the reference modules themselves, imported in the build container
 from ``/root/reference`` by ``oracle/make_golden.py``; the resulting fixtures
 are committed under ``tests/golden/`` and checked by
-``tests/test_oracle_golden.py`` (and live against the reference when
-``/root/reference`` is present).
+``tests/test_oracle_golden.py``.
 """

@@ -9,6 +9,7 @@ TEST INFRASTRUCTURE - see oracle/__init__.py.
 """
 from __future__ import annotations
 
+import io
 import os
 import sys
 
@@ -72,13 +73,43 @@ def golden_hstu(name, V, D, H, blocks, B, L, seed, use_time=True, pass_ts=True):
     grads_ac = {n: (p.grad.clone() if p.grad is not None else torch.zeros_like(p)) for n, p in m.named_parameters()}
     m.eval()
     top = m.predict(ids, ts if pass_ts else None, top_k=10)
-    torch.save(dict(autocast=dict(loss=loss_ac.detach().float(), grads=grads_ac, logits_last=logits_ac.detach().float()[:, -1]),
-                    cfg=dict(num_items=V, embed_dim=D, num_heads=H, num_blocks=blocks, use_temporal_bias=use_time,
-                             pass_ts=pass_ts),
-                    state_dict={k: v.clone() for k, v in m.state_dict().items()},
-                    input_ids=ids, timestamps=ts, targets=tg,
-                    logits=logits.detach(), loss=loss.detach(), grads=grads, top10=top),
-               os.path.join(OUT, name))
+    _save(dict(autocast=dict(loss=loss_ac.detach().float(), grads=grads_ac, logits_last=logits_ac.detach().float()[:, -1]),
+               cfg=dict(num_items=V, embed_dim=D, num_heads=H, num_blocks=blocks, use_temporal_bias=use_time,
+                        pass_ts=pass_ts),
+               state_dict={k: v.clone() for k, v in m.state_dict().items()},
+               input_ids=ids, timestamps=ts, targets=tg,
+               logits=logits.detach(), loss=loss.detach(), grads=grads, top10=top),
+          name, parts=("grads", "autocast"))
+
+
+def _save(d, name, parts=()):
+    """torch.save ``d`` as tests/golden/<name>.  Fixture files stay under 1 MB: a larger one keeps each key in ``parts`` in its own
+    file <stem>.<key>.pt (tests/conftest.py's ``golden`` loader puts them back)."""
+    buf = io.BytesIO()
+    torch.save(d, buf)
+    if buf.tell() > 1_000_000 and parts:
+        for key in parts:
+            torch.save(d.pop(key), os.path.join(OUT, f"{name[:-3]}.{key}.pt"))
+        d["_parts"] = list(parts)
+    torch.save(d, os.path.join(OUT, name))
+
+
+def golden_hstu_fp64(name, seed=3):
+    """The reference HSTU in fp64 (default init, no dropout) on a padded batch with timestamps: logits and loss, for the oracle's
+    1e-12 agreement check.  The parameters are initialised in fp32 and converted, so they are stored in fp32 exactly."""
+    R = ref_loader.ref_hstu()
+    torch.manual_seed(seed)
+    m = R.HSTU(num_items=60, max_seq_len=40, embed_dim=64, num_heads=2, num_blocks=2, dropout=0.0).double()
+    B, L = 3, 37
+    ids = torch.randint(1, 61, (B, L)); ids[0, :11] = 0
+    ts = torch.cumsum(torch.randint(1, 10 ** 6, (B, L)), 1) + 1_300_000_000; ts[ids == 0] = 0
+    tg = torch.randint(1, 61, (B, L))
+    with torch.no_grad():
+        logits, loss = m(ids, ts, tg)
+    sd = {k: v.float() for k, v in m.state_dict().items()}
+    assert all(torch.equal(sd[k].double(), v) for k, v in m.state_dict().items())
+    _save(dict(cfg=dict(num_heads=2, num_blocks=2), state_dict=sd, input_ids=ids, timestamps=ts, targets=tg, logits=logits,
+               loss=loss), name)
 
 
 def golden_hstu_layer(name, D, H, B, L, seed):
@@ -279,6 +310,7 @@ def main():
     golden_hstu("hstu_model_d64h2.pt", V=50, D=64, H=2, blocks=2, B=4, L=24, seed=10)
     golden_hstu("hstu_model_d128h4_nots.pt", V=40, D=128, H=4, blocks=1, B=3, L=17, seed=20, use_time=True, pass_ts=False)
     golden_hstu("hstu_model_notime.pt", V=40, D=64, H=2, blocks=1, B=3, L=9, seed=30, use_time=False)
+    golden_hstu_fp64("hstu_model_fp64.pt")
     golden_hstu_layer("hstu_layer_d64h2_L70.pt", D=64, H=2, B=3, L=70, seed=40)
     golden_hstu_layer("hstu_layer_d64h2_L1.pt", D=64, H=2, B=3, L=1, seed=50)
     golden_sasrec("sasrec_d64h2.pt", V=50, D=64, H=2, blocks=2, F_=256, B=4, L=21, seed=60)

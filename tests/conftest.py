@@ -30,6 +30,10 @@ def golden():
     import torch
 
     def load(name):
-        return torch.load(os.path.join(GOLDEN, name), weights_only=False)
+        g = torch.load(os.path.join(GOLDEN, name), weights_only=False)
+        # a fixture that would exceed 1 MB keeps some top-level entries in side files <stem>.<key>.pt (oracle/make_golden.py)
+        for key in g.pop("_parts", ()):
+            g[key] = torch.load(os.path.join(GOLDEN, f"{name[:-3]}.{key}.pt"), weights_only=False)
+        return g
 
     return load

@@ -71,7 +71,7 @@ def test_head_all_rows_ignored_is_nan_like_the_reference():
     assert torch.isnan(got[0])                       # F.cross_entropy: 0 / 0 valid targets (hstu.py:141-146)
 
 
-def test_head_schedules_agree():
+def test_head_schedules_agree(tmp_path):
     """GRB_CE=store keeps the G' tensor and the TN GEMM for dE (the only schedule at D = 256); GRB_CE=exact is the two-sweep kernel without
     any [T, C] tensor; the default is the one-sweep kernel.  All three must agree at D = 128."""
     code = (
@@ -81,7 +81,7 @@ def test_head_schedules_agree():
         "torch.save(out, sys.argv[1])\n" % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     outs = []
     for mode in ("store", "exact", ""):
-        path = f"/tmp/_head_{mode or 'default'}.pt"
+        path = str(tmp_path / f"head_{mode or 'default'}.pt")
         env = dict(os.environ, GRB_CE=mode)
         if not mode:
             env.pop("GRB_CE")
@@ -119,7 +119,7 @@ def _overflow_case():
     return x, ln_g, ln_b, table, tg
 
 
-def test_one_sweep_range_limit_is_loud_and_exact_mode_has_none():
+def test_one_sweep_range_limit_is_loud_and_exact_mode_has_none(tmp_path):
     """DESIGN 3.3: the one-sweep kernel's exponent shift is max(probe tile, target logit); a class beating both by more than ~98 nats
     overflows that row - the loss comes out non-finite, never silently wrong - and GRB_CE=exact computes the same case exactly."""
     code = (
@@ -129,7 +129,7 @@ def test_one_sweep_range_limit_is_loud_and_exact_mode_has_none():
         "torch.save(out, sys.argv[1])\n" % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     res = {}
     for mode in ("", "exact"):
-        path = f"/tmp/_head_overflow_{mode or 'default'}.pt"
+        path = str(tmp_path / f"head_overflow_{mode or 'default'}.pt")
         env = dict(os.environ, GRB_CE=mode)
         if not mode:
             env.pop("GRB_CE")

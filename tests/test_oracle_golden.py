@@ -1,11 +1,9 @@
-"""The oracle restatement vs the fixtures produced by the UNMODIFIED reference (oracle/make_golden.py),
-and - when /root/reference is present (build container) - vs the live reference in fp64."""
+"""The oracle restatement vs the fixtures produced by the UNMODIFIED reference (oracle/make_golden.py)."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import hstu as oh
-from oracle import ref_loader
 from oracle import rqvae as orq
 from oracle import sasrec as osr
 
@@ -129,19 +127,13 @@ def test_collate_known_answers(golden):
     assert c["timestamps"].tolist() == [[10, 20, 30], [0, 0, 7]]
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted")
-def test_oracle_vs_live_reference_fp64():
-    R = ref_loader.ref_hstu()
-    torch.manual_seed(3)
-    m = R.HSTU(num_items=60, max_seq_len=40, embed_dim=64, num_heads=2, num_blocks=2, dropout=0.0).double()
-    B, L = 3, 37
-    ids = torch.randint(1, 61, (B, L)); ids[0, :11] = 0
-    ts = torch.cumsum(torch.randint(1, 10 ** 6, (B, L)), 1) + 1_300_000_000; ts[ids == 0] = 0
-    tg = torch.randint(1, 61, (B, L))
-    lo, ls = m(ids, ts, tg)
-    sd = {k: v.detach() for k, v in m.state_dict().items()}
-    lo2, ls2 = oh.hstu_forward(ids, ts, tg, sd, 2, 2)
-    assert (lo - lo2).abs().max() < 1e-12 and (ls - ls2).abs() < 1e-12
+def test_oracle_vs_reference_fp64(golden):
+    """The oracle restatement in fp64 reproduces the logits and loss of the unmodified reference HSTU run in fp64."""
+    g = golden("hstu_model_fp64.pt")
+    sd = {k: v.double() for k, v in g["state_dict"].items()}
+    lo, ls = oh.hstu_forward(g["input_ids"], g["timestamps"], g["targets"], sd, g["cfg"]["num_heads"], g["cfg"]["num_blocks"])
+    assert lo.dtype == g["logits"].dtype == torch.float64
+    assert (lo - g["logits"]).abs().max() < 1e-12 and (ls - g["loss"]).abs() < 1e-12
 
 
 @pytest.mark.parametrize("name", ["tiger_decode_trie.pt", "tiger_decode_notrie.pt"])
