@@ -671,13 +671,16 @@ __global__ void __launch_bounds__(256) ce_fwd_bwd_vec_kernel(bf16* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------------ fused Adam (torch.optim.Adam semantics)
-// state[0] = step (as float), state[1] = 1 - beta1^step, state[2] = 1 - beta2^step ; ticked on device so a CUDA graph replays correctly
+// state[0] = step (as float), state[1] = 1 - beta1^step, state[2] = 1 - beta2^step ; ticked on device so a CUDA graph replays correctly.
+// The powers are taken in double: under --use_fast_math powf is exp2(step * log2(beta)) on the approximate MUFU units, and the
+// cancellation in 1 - beta2^step (beta2 = 0.999) magnified their error to 6e-5 of the bias correction on a B200 - every update of the
+// first steps was off by the same factor.  Double arithmetic is not affected by fast math.
 __global__ void adam_tick_kernel(float* state, float beta1, float beta2) {
     pdl_wait();
     float step = state[0] + 1.f;
     state[0] = step;
-    state[1] = 1.f - powf(beta1, step);
-    state[2] = 1.f - powf(beta2, step);
+    state[1] = (float)(1.0 - pow((double)beta1, (double)step));
+    state[2] = (float)(1.0 - pow((double)beta2, (double)step));
 }
 struct AdamArgs {
     float* p; float* g; float* m; float* v; bf16* p_bf16;  // p_bf16 nullable

@@ -9,12 +9,19 @@ TEST INFRASTRUCTURE - see oracle/__init__.py.
 from __future__ import annotations
 
 import math
-from typing import Dict, Optional, Tuple
+from typing import Callable, Dict, Optional, Tuple
 
 import torch
 import torch.nn.functional as F
 
 Params = Dict[str, torch.Tensor]
+# drop(name, t) -> t': a dropout site of the reference, by name.  Tests pass one that multiplies by a known mask (kept elements
+# scaled, dropped ones 0) so the oracle reproduces a training-mode forward; None is eval mode.
+Drop = Callable[[str, torch.Tensor], torch.Tensor]
+
+
+def _no_drop(name: str, t: torch.Tensor) -> torch.Tensor:
+    return t
 
 
 # --------------------------------------------------------------------------- buckets
@@ -78,8 +85,13 @@ def hstu_layer_forward(
     num_position_buckets: int = 32,
     max_position_distance: int = 128,
     return_intermediates: bool = False,
+    drop: Optional[Drop] = None,
 ):
-    """One HSTU block, dropout = 0.  Follows genrec/models/hstu.py:222-280 (SURVEY Appendix A)."""
+    """One HSTU block.  Follows genrec/models/hstu.py:222-280 (SURVEY Appendix A).
+
+    ``drop(name, t)`` stands for the reference's nn.Dropout at the three places it sits in a block (None = eval mode):
+    ``{prefix}gate`` (:275), ``{prefix}ffn_hid`` (:212) and ``{prefix}ffn_out`` (:214)."""
+    drop = drop or _no_drop
     B, L, D = x.shape
     H, dh = num_heads, D // num_heads
     g = lambda k: p[prefix + k]
@@ -103,10 +115,10 @@ def hstu_layer_forward(
     O = (A @ V).transpose(1, 2).reshape(B, L, D)                                  # :266-267
 
     N = _ln(O, g("attn_norm.weight"), g("attn_norm.bias"), 1e-5)                 # :271
-    x1 = x + N * U                                                                # :272-275
+    x1 = x + drop(prefix + "gate", N * U)                                         # :272-275
     xn = _ln(x1, g("ffn_norm.weight"), g("ffn_norm.bias"), 1e-5)                 # :278
-    hid = F.silu(xn @ g("ffn.0.weight").T + g("ffn.0.bias"))                     # :210-211
-    y = x1 + hid @ g("ffn.3.weight").T + g("ffn.3.bias")                         # :213, :278
+    hid = drop(prefix + "ffn_hid", F.silu(xn @ g("ffn.0.weight").T + g("ffn.0.bias")))   # :210-212
+    y = x1 + drop(prefix + "ffn_out", hid @ g("ffn.3.weight").T + g("ffn.3.bias"))     # :213-214, :278
     if return_intermediates:
         return y, dict(P=proj, S=S, A=A, O=O, N=N, x1=x1, xn=xn, hid=hid)
     return y
@@ -122,14 +134,17 @@ def hstu_forward(
     use_temporal_bias: bool = True,
     num_position_buckets: int = 32,
     max_position_distance: int = 128,
+    drop: Optional[Drop] = None,
 ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
-    """Whole model, dropout = 0.  Follows genrec/models/hstu.py:99-148."""
+    """Whole model.  Follows genrec/models/hstu.py:99-148.  ``drop``: see ``hstu_layer_forward``; the embedding's is ``emb`` (:128)."""
+    drop = drop or _no_drop
     padding_mask = input_ids == 0                                                 # :124
     E = p["item_embedding.weight"]
     x = F.embedding(input_ids, E, padding_idx=0)      # :127 (+ :62 padding_idx: no gather-grad into row 0)
+    x = drop("emb", x)                                                            # :128
     for i in range(num_blocks):                                                   # :131-132
         x = hstu_layer_forward(x, padding_mask, timestamps, p, f"layers.{i}.", num_heads,
-                               use_temporal_bias, num_position_buckets, max_position_distance)
+                               use_temporal_bias, num_position_buckets, max_position_distance, drop=drop)
     x = _ln(x, p["final_norm.weight"], p["final_norm.bias"], 1e-5)               # :134
     logits = x @ E.T                                                              # :137
     loss = None

@@ -175,6 +175,84 @@ def golden_sasrec(name, V, D, H, blocks, F_, B, L, seed):
                os.path.join(OUT, name))
 
 
+def _pin_dropout(model, sites, seed, p):
+    """Replace the output of every nn.Dropout of ``model`` by ``input * mask`` through forward hooks (the reference source stays
+    untouched).  ``sites(module_name, call_index) -> oracle site name``: a module that runs more than once per forward (SASRec's
+    PointWiseFeedForward) is told apart by call order.  The keep masks are drawn once per site name (first forward) and replayed
+    afterwards; returns (masks, reset) - call reset() before each forward."""
+    g = torch.Generator().manual_seed(seed)
+    masks, calls = {}, {}
+
+    def hook(mod_name):
+        def f(mod, inp, out):
+            k = calls.get(mod_name, 0)
+            calls[mod_name] = k + 1
+            site = sites(mod_name, k)
+            if site not in masks:
+                masks[site] = torch.rand(inp[0].shape, generator=g) >= p
+            return inp[0] * (masks[site].to(inp[0].dtype) / (1 - p))
+        return f
+
+    for n, mod in model.named_modules():
+        if isinstance(mod, torch.nn.Dropout):
+            mod.register_forward_hook(hook(n))
+    return masks, calls.clear
+
+
+def golden_hstu_dropout(name, V=50, D=64, H=2, blocks=2, B=3, L=20, p=0.2, seed=110):
+    """The reference HSTU in train mode with every nn.Dropout pinned to a recorded mask: loss, logits and every gradient, plus the
+    masks (bool, True = kept; a kept element is scaled by 1 / (1 - p)) under the oracle's site names."""
+    R = ref_loader.ref_hstu()
+    torch.manual_seed(seed)
+    m = R.HSTU(num_items=V, max_seq_len=L, embed_dim=D, num_heads=H, num_blocks=blocks, dropout=p)
+    _perturb(m, seed + 1)
+    m.train()
+    names = {"emb_dropout": "emb"}
+    for i in range(blocks):
+        names.update({f"layers.{i}.dropout": f"layers.{i}.gate", f"layers.{i}.ffn.2": f"layers.{i}.ffn_hid",
+                      f"layers.{i}.ffn.4": f"layers.{i}.ffn_out"})
+    masks, reset = _pin_dropout(m, lambda n, k: names[n], seed + 3, p)
+    ids, ts, tg = _batch(B, L, V, seed + 2)
+    reset()
+    logits, loss = m(ids, ts, tg)
+    loss.backward()
+    assert sorted(masks) == sorted(names.values())
+    _save(dict(cfg=dict(num_heads=H, num_blocks=blocks, p=p), state_dict={k: v.clone() for k, v in m.state_dict().items()},
+               input_ids=ids, timestamps=ts, targets=tg, masks=masks, logits=logits.detach(), loss=loss.detach(),
+               grads={n: q.grad.clone() for n, q in m.named_parameters()}), name)
+
+
+def golden_sasrec_dropout(name, V=50, D=64, H=2, blocks=2, F_=128, B=3, L=20, p=0.2, seed=120):
+    """As golden_hstu_dropout, for SASRec: embedding, attention weights, and the two calls of each block's FFN dropout."""
+    S = ref_loader.ref_sasrec()
+    torch.manual_seed(seed)
+    m = S.SASRec(num_items=V, max_seq_len=L, embed_dim=D, num_heads=H, num_blocks=blocks, ffn_dim=F_, dropout=p)
+    g = torch.Generator().manual_seed(seed + 1)
+    with torch.no_grad():
+        for n, q in m.named_parameters():
+            if n.endswith("bias"):
+                q.copy_(0.1 * torch.randn(q.shape, generator=g))
+            elif "norm" in n:
+                q.add_(0.1 * torch.randn(q.shape, generator=g))
+    m.train()
+
+    def site(n, k):
+        if n == "emb_dropout":
+            return "emb"
+        blk = n.split(".attention.")[0].split(".ffn.")[0] + "."
+        return blk + ("attn" if n.endswith("attention.dropout") else ("ffn_hid", "ffn_out")[k])
+
+    masks, reset = _pin_dropout(m, site, seed + 3, p)
+    ids, _, tg = _batch(B, L, V, seed + 2)
+    reset()
+    logits, loss = m(ids, tg)
+    loss.backward()
+    assert len(masks) == 1 + 3 * blocks
+    _save(dict(cfg=dict(num_heads=H, num_blocks=blocks, p=p), state_dict={k: v.clone() for k, v in m.state_dict().items()},
+               input_ids=ids, targets=tg, masks=masks, logits=logits.detach(), loss=loss.detach(),
+               grads={n: q.grad.clone() for n, q in m.named_parameters()}), name)
+
+
 def golden_rqvae(name, seed, N=300, levels=3, K=256, D=32):
     ns = ref_loader.ref_genrec_package()
     rq = ns.rqvae
@@ -314,6 +392,8 @@ def main():
     golden_hstu_layer("hstu_layer_d64h2_L70.pt", D=64, H=2, B=3, L=70, seed=40)
     golden_hstu_layer("hstu_layer_d64h2_L1.pt", D=64, H=2, B=3, L=1, seed=50)
     golden_sasrec("sasrec_d64h2.pt", V=50, D=64, H=2, blocks=2, F_=256, B=4, L=21, seed=60)
+    golden_hstu_dropout("hstu_dropout.pt")
+    golden_sasrec_dropout("sasrec_dropout.pt")
     golden_rqvae("rqvae_3x256x32.pt", seed=70)
     golden_kats("kats.pt")
     golden_t5_attention("t5_attention.pt", seed=100)

@@ -2,6 +2,8 @@
 import pytest
 import torch
 
+from tests.util import drop_mask
+
 pytestmark = pytest.mark.gpu
 
 
@@ -99,7 +101,7 @@ def test_dropout_masks_agree_between_forward_and_backward(p):
     c3 = Fn.cast_rows_bf16(torch.ones(T, K, device=dev), p=p, seed=seed + 1, site=site + 1)
     assert not torch.equal(c2 == 0, c == 0) and not torch.equal(c3 == 0, c == 0)
     # the mask is the documented pure function of (seed, site, row, column): bit-exact against the numpy restatement
-    assert torch.equal((c == 0).cpu(), torch.from_numpy(_np_drop_mask(T, K, p, seed, site + 1)))
+    assert torch.equal((c == 0).cpu(), torch.from_numpy(drop_mask(range(T), range(K), p, seed, site + 1)))
     # rows and columns are decorrelated: cross-correlations are those of an ideal generator
     Tm, Dm = 512, 1024
     m = (Fn.cast_rows_bf16(torch.ones(Tm, Dm, device=dev), p=p, seed=seed, site=9) == 0).double()
@@ -114,26 +116,3 @@ def test_dropout_masks_agree_between_forward_and_backward(p):
     assert abs((m[1:] * m[:-1]).mean().item() - p * p) < 0.005
     assert abs((m[:, 1:] * m[:, :-1]).mean().item() - p * p) < 0.005
 
-
-def _np_drop_mask(T, D, p, seed, site):
-    """numpy restatement of genrec_b200/csrc/common.cuh Dropout (row keys + pair hash); True = dropped."""
-    import numpy as np
-    u = np.uint32
-    k0 = u((seed & 0xffffffff) ^ ((site * 0x9E3779B1) & 0xffffffff))
-    k1 = u(((seed >> 32) + 0x7F4A7C15) & 0xffffffff)
-    row = np.arange(T, dtype=np.uint32)[:, None]
-    cp = np.arange(D // 2, dtype=np.uint32)[None, :]
-    with np.errstate(over="ignore"):
-        ka = (row ^ k1) * u(0x9E3779B1)
-        ka = ka ^ (ka >> u(16))
-        b = ka * u(0x846CA68B)
-        kb = k0 ^ (b ^ (b >> u(15)))
-        x = (cp ^ kb) * u(0x7FEB352D)
-        x = x ^ (x >> u(15))
-        x = (x ^ ka) * u(0x846CA68B)
-        x = x ^ (x >> u(16))
-    t = u(int(p * 65536.0 + 0.5))
-    m = np.empty((T, D), dtype=bool)
-    m[:, 0::2] = (x & u(0xffff)) < t
-    m[:, 1::2] = (x >> u(16)) < t
-    return m

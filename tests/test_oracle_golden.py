@@ -99,6 +99,36 @@ def test_sasrec(golden):
         torch.testing.assert_close(p["blocks.0.attention." + n].grad, gr, rtol=1e-4, atol=1e-4)
 
 
+@pytest.mark.parametrize("name", ["hstu_dropout.pt", "sasrec_dropout.pt"])
+def test_dropout_sites_vs_reference_golden(golden, name):
+    """Training mode: the unmodified reference with every nn.Dropout pinned to a recorded mask (oracle/make_golden.py) against the
+    oracle's ``drop`` hook fed the same masks - each hook sits where the reference applies its dropout, and every site is used."""
+    g = golden(name)
+    cfg = g["cfg"]
+    p = _req(g["state_dict"])
+    used = []
+
+    def drop(site, t):
+        used.append(site)
+        return t * (g["masks"][site].to(t.dtype) / (1 - cfg["p"]))
+
+    if name.startswith("hstu"):
+        logits, loss = oh.hstu_forward(g["input_ids"], g["timestamps"], g["targets"], p, cfg["num_heads"], cfg["num_blocks"], drop=drop)
+    else:
+        logits, loss = osr.sasrec_forward(g["input_ids"], g["targets"], p, cfg["num_heads"], cfg["num_blocks"], drop=drop)
+    assert sorted(used) == sorted(g["masks"])
+    torch.testing.assert_close(logits, g["logits"], rtol=1e-5, atol=5e-5)
+    torch.testing.assert_close(loss, g["loss"], rtol=1e-6, atol=1e-6)
+    loss.backward()
+    for n, gr in g["grads"].items():
+        got = p[n].grad if p[n].grad is not None else torch.zeros_like(p[n])
+        torch.testing.assert_close(got, gr, rtol=5e-4, atol=5e-6, msg=lambda m: f"{n}: {m}")
+    # the masks really drop: without them the oracle is far from the recording
+    lo0, _ = (oh.hstu_forward(g["input_ids"], g["timestamps"], None, g["state_dict"], cfg["num_heads"], cfg["num_blocks"])
+              if name.startswith("hstu") else osr.sasrec_forward(g["input_ids"], None, g["state_dict"], cfg["num_heads"], cfg["num_blocks"]))
+    assert (lo0 - g["logits"]).abs().max() > 1e-2 * g["logits"].abs().max()
+
+
 def test_rqvae(golden):
     g = golden("rqvae_3x256x32.pt")
     sd = g["state_dict"]
