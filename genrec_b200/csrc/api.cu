@@ -17,12 +17,10 @@
 #include "common.cuh"
 #include "dp_adam.cuh"
 #include "exact_f32.cuh"
-#include "gemm.cuh"
 #include "rowwise.cuh"
 #include "rq_argmin.cuh"
 #include "tc_gemm.cuh"
 #include "tc_ce.cuh"
-#include "tc_ffn.cuh"
 #include "tc_tn_group.cuh"
 #include <cstdlib>
 
@@ -91,25 +89,9 @@ int row_grid(int T) {
     int cap = sm_count() * 8;
     return need < cap ? (need < 1 ? 1 : need) : cap;
 }
-int splitk_for(int M, int N, int K) {
-    int tiles = ((M + GEMM_BM - 1) / GEMM_BM) * ((N + GEMM_BN - 1) / GEMM_BN);
-    int want = (2 * sm_count() + tiles - 1) / tiles;
-    int kt = (K + GEMM_BK - 1) / GEMM_BK;
-    int maxs = kt / 4 > 0 ? kt / 4 : 1;  // at least 4 k-tiles per split
-    return want < 1 ? 1 : (want > maxs ? maxs : want);
-}
 
 
-// ---- GEMM dispatch: tcgen05/TMA path (default) or the first-generation mma.sync path (GRB_GEMM=mma, kept as an on-device
-//      cross-check).  Operand majors: *_MN = 0 -> K contiguous, 1 -> M/N contiguous (see tc_gemm.cuh / gemm.cuh).
-bool use_tc() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GRB_GEMM");
-        v = (e && strcmp(e, "mma") == 0) ? 0 : 1;
-    }
-    return v == 1;
-}
+// ---- GEMM wrappers over the tcgen05/TMA kernel.  Operand majors: *_MN = 0 -> K contiguous, 1 -> M/N contiguous (see tc_gemm.cuh).
 int tn_splits(int M, int N, int K) {
     int tiles = ((M + TC_BM - 1) / TC_BM) * ((N + TC_BN - 1) / TC_BN);
     int want = (sm_count() + tiles - 1) / tiles;
@@ -120,50 +102,32 @@ int tn_splits(int M, int N, int K) {
 // z = x W^T + b ; act: 0 none, 1 silu, 2 relu   (NT)
 cudaError_t gemm_bias_act(int act, const bf16* x, const bf16* w, const float* bias, bf16* z, bf16* a, int M, int N, int K, const Dropout& drop,
                           cudaStream_t st) {
-    if (use_tc()) {
-        if (act == 0) return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<0>{bias, N, drop}, z, nullptr, N, sm_count(), st);
-        if (act == 1) return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<1>{bias, N, drop}, z, a, N, sm_count(), st);
-        return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<2>{bias, N, drop}, z, a, N, sm_count(), st);
-    }
-    if (act == 0) return launch_gemm<0, 0>(x, w, M, N, K, K, K, 1, EpiBiasBf16{bias, z, N}, st);
-    if (act == 1) return launch_gemm<0, 0>(x, w, M, N, K, K, K, 1, EpiBiasSilu{bias, z, a, N, drop}, st);
-    return launch_gemm<0, 0>(x, w, M, N, K, K, K, 1, EpiBiasRelu{bias, z, a, N, drop}, st);
+    if (act == 0) return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<0>{bias, N, drop}, z, nullptr, N, sm_count(), st);
+    if (act == 1) return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<1>{bias, N, drop}, z, a, N, sm_count(), st);
+    return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasAct<2>{bias, N, drop}, z, a, N, sm_count(), st);
 }
 // y = res + drop(x W^T + b) (* row_scale)   (NT)
 cudaError_t gemm_bias_res(const bf16* x, const bf16* w, const float* bias, const float* res, const float* row_scale, float* y, int M, int N,
                           int K, const Dropout& drop, cudaStream_t st) {
-    if (use_tc()) return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasResidual{bias, res, row_scale, N, drop}, y, nullptr, N, sm_count(), st);
-    return launch_gemm<0, 0>(x, w, M, N, K, K, K, 1, EpiBiasResidual{bias, res, y, row_scale, N, drop}, st);
+    return launch_tc_gemm<0, 0>(x, w, M, N, K, K, K, 1, TcEpiBiasResidual{bias, res, row_scale, N, drop}, y, nullptr, N, sm_count(), st);
 }
 // g[M,N] = dropmask(dy[M,K] W[K,N]) * act'(z)   (NN) ; act 1 silu, 2 relu
 cudaError_t gemm_dact(int act, const bf16* dy, const bf16* w, const bf16* z, bf16* g, int M, int N, int K, const Dropout& drop, cudaStream_t st) {
-    if (use_tc()) {
-        if (act == 1) return launch_tc_gemm<0, 1>(dy, w, M, N, K, K, N, 1, TcEpiDAct<1>{z, N, drop}, g, nullptr, N, sm_count(), st);
-        return launch_tc_gemm<0, 1>(dy, w, M, N, K, K, N, 1, TcEpiDAct<2>{z, N, drop}, g, nullptr, N, sm_count(), st);
-    }
-    if (act == 1) return launch_gemm<0, 1>(dy, w, M, N, K, K, N, 1, EpiDAct<0>{z, g, N, drop}, st);
-    return launch_gemm<0, 1>(dy, w, M, N, K, K, N, 1, EpiDAct<1>{z, g, N, drop}, st);
+    if (act == 1) return launch_tc_gemm<0, 1>(dy, w, M, N, K, K, N, 1, TcEpiDAct<1>{z, N, drop}, g, nullptr, N, sm_count(), st);
+    return launch_tc_gemm<0, 1>(dy, w, M, N, K, K, N, 1, TcEpiDAct<2>{z, N, drop}, g, nullptr, N, sm_count(), st);
 }
 // out[M,N] fp32 = scale * A[M,K] B[K,N] (+ res)   (NN)
 cudaError_t gemm_nn_f32(const bf16* A, const bf16* B, float* out, const float* res, float scale, int M, int N, int K, int lda, int ldb,
                         cudaStream_t st) {
-    if (use_tc()) return launch_tc_gemm<0, 1>(A, B, M, N, K, lda, ldb, 1, TcEpiF32{res, N, scale}, out, nullptr, N, sm_count(), st);
-    return launch_gemm<0, 1>(A, B, M, N, K, lda, ldb, 1, EpiF32{out, res, N, scale}, st);
+    return launch_tc_gemm<0, 1>(A, B, M, N, K, lda, ldb, 1, TcEpiF32{res, N, scale}, out, nullptr, N, sm_count(), st);
 }
 // out[M,N] fp32 += A^T B with A stored [K,M], B stored [K,N]   (TN, split-K, atomics)
 cudaError_t gemm_tn_atomic(const bf16* A, const bf16* B, float* out, int M, int N, int K, int lda, int ldb, cudaStream_t st) {
-    if (use_tc()) return launch_tc_gemm<1, 1>(A, B, M, N, K, lda, ldb, tn_splits(M, N, K), TcEpiAtomicF32{out, N, 1.f}, nullptr, nullptr, 0, sm_count(), st);
-    return launch_gemm<1, 1>(A, B, M, N, K, lda, ldb, splitk_for(M, N, K), EpiAtomicF32{out, N, 1.f}, st);
-}
-// out[M,N] bf16 (leading dim ldo) = A[M,K] B[N,K]^T   (NT)
-cudaError_t gemm_nt_bf16(const bf16* A, const bf16* B, bf16* out, int ldo, int M, int N, int K, cudaStream_t st) {
-    if (use_tc()) return launch_tc_gemm<0, 0>(A, B, M, N, K, K, K, 1, TcEpiBf16{}, out, nullptr, ldo, sm_count(), st);
-    return launch_gemm<0, 0>(A, B, M, N, K, K, K, 1, EpiBf16{out, ldo}, st);
+    return launch_tc_gemm<1, 1>(A, B, M, N, K, lda, ldb, tn_splits(M, N, K), TcEpiAtomicF32{out, N, 1.f}, nullptr, nullptr, 0, sm_count(), st);
 }
 // out[M,N] fp32 (leading dim N, any parity) = A B^T   (NT)
 cudaError_t gemm_nt_f32_plain(const bf16* A, const bf16* B, float* out, int M, int N, int K, cudaStream_t st) {
-    if (use_tc()) return launch_tc_gemm<0, 0>(A, B, M, N, K, K, K, 1, TcEpiF32Plain{out, N}, nullptr, nullptr, 0, sm_count(), st);
-    return launch_gemm<0, 0>(A, B, M, N, K, K, K, 1, EpiF32Scalar{out, N, N}, st);
+    return launch_tc_gemm<0, 0>(A, B, M, N, K, K, K, 1, TcEpiF32Plain{out, N}, nullptr, nullptr, 0, sm_count(), st);
 }
 
 // ---- carved layouts ------------------------------------------------------------------------------------------
@@ -526,14 +490,6 @@ int cast_colsum(const float* in, bf16* out, int T, int D, const Dropout& drop, f
     GRB_CUDA(cudaGetLastError());
     return 0;
 }
-// GRB_FFN_FUSED=1 routes the forward FFN through the single fused kernel of tc_ffn.cuh.  Off by default: at cfg-2 it
-// measures 47 us per layer against 43 us for the two separate GEMM launches (its 16 epilogue warps walk the phases of a
-// chunk in lock-step); it is the first building block of the fused layer kernel and is kept bit-compatible and tested.
-// Read on every call so that a test can flip it.
-bool ffn_fused() {
-    const char* e = getenv("GRB_FFN_FUSED");
-    return e != nullptr && e[0] == '1';
-}
 int colsum(const bf16* in, int T, int N, int ld, float* out, cudaStream_t st) {
     if (N % 8 != 0 || ld % 8 != 0) return fail(GRB_EINVAL, "colsum needs N and ld to be multiples of 8");
     int cx = (N + 255) / 256;
@@ -612,15 +568,6 @@ int grb_hstu_layer_forward(const grb_hstu_dims* d, const grb_hstu_layer_params* 
                         make_dropout(d->dropout_p, d->seed, site_of(d->layer_index, SITE_GATE), d->seed_dev)};
         GRB_ROW_DISPATCH(D, ln_gate_fwd_kernel, a, T, st);
     }
-    // 5 + 6 in one kernel (tc_ffn.cuh): h is written once for the backward and never re-read in the forward
-    if (use_tc() && ffn_fused() && (D == 64 || D == 128)) {
-        FfnEpiArgs ea{p->ffn1_b, p->ffn2_b, sv.x1, sv.z1, y,
-                      make_dropout(d->dropout_p, d->seed, site_of(d->layer_index, SITE_FFN_HID), d->seed_dev),
-                      make_dropout(d->dropout_p, d->seed, site_of(d->layer_index, SITE_FFN_OUT), d->seed_dev)};
-        if (D == 64) GRB_CUDA(launch_tc_ffn_fwd<1>(sv.xn, (const bf16*)p->ffn1_w, (const bf16*)p->ffn2_w, sv.hact, T, ea, sm_count(), st));
-        else GRB_CUDA(launch_tc_ffn_fwd<2>(sv.xn, (const bf16*)p->ffn1_w, (const bf16*)p->ffn2_w, sv.hact, T, ea, sm_count(), st));
-        return 0;
-    }
     // 5. h = drop(silu(xn W1^T + b1))                                                        (hstu.py:210-212)
     {
         GRB_CUDA(gemm_bias_act(1, sv.xn, (const bf16*)p->ffn1_w, p->ffn1_b, sv.z1, sv.hact, T, 4 * D, D,
@@ -653,21 +600,15 @@ int grb_hstu_layer_backward(const grb_hstu_dims* d, const grb_hstu_layer_params*
     // FFN second linear
     GRB_TRY(cast_colsum(dy, w.dyb, T, D, drop_out, g->ffn2_b, st));   // dyb = bf16(dropmask(dy)) ; db2 += column sums
     {
-        if (!use_tc()) GRB_CUDA(gemm_tn_atomic(w.dyb, sv.hact, g->ffn2_w, D, 4 * D, T, D, 4 * D, st));  // dW2[D,4D] += dyb^T h
-    }
-    {
         GRB_CUDA(gemm_dact(1, w.dyb, (const bf16*)p->ffn2_w, sv.z1, w.dz1, T, 4 * D, D, drop_hid, st));  // dz1 = dropmask(dyb W2) * silu'(z1)
     }
     // FFN first linear
     // bias gradients are off the critical path too: with deferred weight gradients the column sums run beside the main chain
     auto colsum_maybe_deferred = [&](const bf16* in, float* out) -> int {
-        if (use_tc() && g_defer_on) return defer_run(st, [&](cudaStream_t side) -> int { return colsum(in, T, 4 * D, 4 * D, out, side); });
+        if (g_defer_on) return defer_run(st, [&](cudaStream_t side) -> int { return colsum(in, T, 4 * D, 4 * D, out, side); });
         return colsum(in, T, 4 * D, 4 * D, out, st);
     };
     GRB_TRY(colsum_maybe_deferred(w.dz1, g->ffn1_b));
-    {
-        if (!use_tc()) GRB_CUDA(gemm_tn_atomic(w.dz1, sv.xn, g->ffn1_w, 4 * D, D, T, 4 * D, D, st));  // dW1[4D,D] += dz1^T xn
-    }
     {
         GRB_CUDA(gemm_nn_f32(w.dz1, (const bf16*)p->ffn1_w, w.dxn, nullptr, 1.f, T, D, 4 * D, 4 * D, D, st));  // dxn = dz1 W1
     }
@@ -695,12 +636,9 @@ int grb_hstu_layer_backward(const grb_hstu_dims* d, const grb_hstu_layer_params*
     // projection
     GRB_TRY(colsum_maybe_deferred(w.dzp, g->proj_b));
     {
-        if (!use_tc()) GRB_CUDA(gemm_tn_atomic(w.dzp, sv.xb, g->proj_w, 4 * D, D, T, 4 * D, D, st));  // dWp[4D,D] += dzp^T xb
-    }
-    {
         GRB_CUDA(gemm_nn_f32(w.dzp, (const bf16*)p->proj_w, dx, w.dx1, 1.f, T, D, 4 * D, 4 * D, D, st));  // dx = dx1 + dzp Wp
     }
-    if (use_tc()) {
+    {
         // the three weight gradients of the layer in ONE grouped launch: dW2 += dyb^T h, dW1 += dz1^T xn, dWp += dzp^T xb
         TnSpec specs[3] = {{w.dyb, sv.hact, g->ffn2_w, D, 4 * D, T, D, 4 * D, 4 * D},
                            {w.dz1, sv.xn, g->ffn1_w, 4 * D, D, T, 4 * D, D, D},
@@ -878,7 +816,7 @@ int grb_head_loss_forward_backward(const float* x, const float* ln_g, const floa
     const bool count_aside = g_defer_on;
     // D <= 128: no [T, C] tensor reaches HBM - dX' accumulates in TMEM beside the CE sweep and dE comes from a class-stationary pass
     // that recomputes G.  D = 256 (or GRB_CE=store): G' is stored and dE is a TN GEMM.
-    const bool keep_g = use_tc() && D <= 128 && want_grad && !ce_store_forced();
+    const bool keep_g = D <= 128 && want_grad && !ce_store_forced();
     const int ce_mode = keep_g ? ce_mode_env() : (int)CE_STORE_G;
     auto count = [&](cudaStream_t s_) -> int {
         launch_k(ce_count_kernel, 1, 1024, 0, s_, reinterpret_cast<const long long*>(targets), T, h.scal, loss);
@@ -893,22 +831,15 @@ int grb_head_loss_forward_backward(const float* x, const float* ln_g, const floa
     if (count_aside) GRB_TRY(join_pending(st));
     else GRB_TRY(count(st));
     bool fused_dx = false;
-    if (use_tc()) {
+    {
         // fused: logits are never materialised; (D <= 128) h.dxf = G' E, and h.logits receives G' only when a dE GEMM needs it
         const long long* tg = reinterpret_cast<const long long*>(targets);                                  // (hstu.py:137-146)
         const bf16* tb = (const bf16*)table_bf16;
         if (D == 64) GRB_CUDA(launch_tc_ce<1>(h.xf, tb, h.logits, ce_mode, T, C, h.ldl, tg, h.scal, h.row_sums, h.row_stats, h.dxf, &fused_dx, h.ce_scratch, sm_count(), st));
         else if (D == 128) GRB_CUDA(launch_tc_ce<2>(h.xf, tb, h.logits, ce_mode, T, C, h.ldl, tg, h.scal, h.row_sums, h.row_stats, h.dxf, &fused_dx, h.ce_scratch, sm_count(), st));
         else GRB_CUDA(launch_tc_ce<4>(h.xf, tb, h.logits, CE_STORE_G, T, C, h.ldl, tg, h.scal, h.row_sums, h.row_stats, h.dxf, &fused_dx, h.ce_scratch, sm_count(), st));
-    } else {
-    GRB_CUDA(gemm_nt_bf16(h.xf, (const bf16*)table_bf16, h.logits, h.ldl, T, C, D, st));  // logits = xf E^T   (hstu.py:137)
-    if (h.ldl / 8 <= 256 * 8)
-        launch_k(ce_fwd_bwd_vec_kernel<8>, T, 256, 0, st, h.logits, h.ldl, C, reinterpret_cast<const long long*>(targets), h.scal, loss, want_grad ? 1 : 0);
-    else
-        launch_k(ce_fwd_bwd_kernel, T, 256, 0, st, h.logits, h.ldl, C, reinterpret_cast<const long long*>(targets), h.scal, loss, want_grad ? 1 : 0);
-    GRB_CUDA(cudaGetLastError());
     }
-    if (use_tc()) {
+    {
         // normalisation pass of the fused CE (rowwise.cuh ce_finish_kernel): loss, and - with gradients - dxf, x / sum_row, the one-hot
         // term of dE.  Without the dX fusion (D = 256) dxf' = G' E comes from a GEMM first.
         if (want_grad && !fused_dx) GRB_CUDA(gemm_nn_f32(h.logits, (const bf16*)table_bf16, h.dxf, nullptr, 1.f, T, D, C, h.ldl, D, st));
@@ -921,9 +852,6 @@ int grb_head_loss_forward_backward(const float* x, const float* ln_g, const floa
     }
     if (!want_grad) return 0;
     {
-        if (!use_tc()) GRB_CUDA(gemm_nn_f32(h.logits, (const bf16*)table_bf16, h.dxf, nullptr, 1.f, T, D, C, h.ldl, D, st));  // dxf = dlogits E
-    }
-    {
         if (keep_g) {
             // dE[C,D] += G^T xf with G recomputed class block by class block (tc_ce.cuh CE_ACCUM_T); off the critical path like the
             // other weight gradients
@@ -934,7 +862,7 @@ int grb_head_loss_forward_backward(const float* x, const float* ln_g, const floa
             };
             if (g_defer_on) GRB_TRY(defer_run(st, accum));
             else GRB_TRY(accum(st));
-        } else if (use_tc()) {
+        } else {
             TnSpec spec{h.logits, h.xs, dtable, C, D, T, h.ldl, D, D};  // dE[C,D] += G'^T (xf / sum_row) = dlogits^T xf
             if (g_defer_on) {
                 GRB_TRY(defer_run(st, [&](cudaStream_t side) -> int {
@@ -944,8 +872,6 @@ int grb_head_loss_forward_backward(const float* x, const float* ln_g, const floa
             } else {
                 GRB_CUDA(launch_tc_tn_group(&spec, 1, sm_count(), st));
             }
-        } else {
-            GRB_CUDA(gemm_tn_atomic(h.logits, h.xf, dtable, C, D, T, h.ldl, D, st));
         }
     }
     {

@@ -1,5 +1,5 @@
 // genrec_b200 - row-wise (per token) kernels: LayerNorm / gate / residual forward+backward, casts, column sums,
-// embedding gather/scatter, cross-entropy over bf16 logits, fused Adam.  HBM-bound; one warp per token row,
+// embedding gather/scatter, the row passes of the fused cross-entropy, fused Adam.  HBM-bound; one warp per token row,
 // 8-byte (bf16x4 / float2) vector accesses, D % 64 == 0, D <= 512.
 #pragma once
 #include "common.cuh"
@@ -482,7 +482,7 @@ __global__ void __launch_bounds__(ROW_THREADS) embed_bwd_kernel(EmbedBwdArgs a) 
     }
 }
 
-// ------------------------------------------------------------------------------------------------ cross entropy on bf16 logits
+// ------------------------------------------------------------------------------------------------ fused CE: target count
 // count = #(targets != 0)  -> inv_count (0 if none); loss <- 0, or NaN when no target is valid (F.cross_entropy's 0 / 0 mean,
 // hstu.py:141-146; the gradients of such a batch are zero here, NaN in the reference)
 __global__ void ce_count_kernel(const long long* __restrict__ tg, int T, float* __restrict__ inv_count, float* __restrict__ loss) {
@@ -507,166 +507,6 @@ __global__ void ce_count_kernel(const long long* __restrict__ tg, int T, float* 
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += red[w];
         *inv_count = s > 0 ? 1.f / (float)s : 0.f;
         *loss = s > 0 ? 0.f : __int_as_float(0x7fc00000);
-    }
-}
-// one CTA per row: loss += (lse - logit[target]) * inv_count ; logits <- (softmax - onehot) * inv_count  (0 for ignored rows)
-// pad columns [C, ld) are written with zeros.   (hstu.py:141-146, ignore_index = 0, class 0 stays in the denominator)
-__global__ void __launch_bounds__(256) ce_fwd_bwd_kernel(bf16* __restrict__ logits, int ld, int C, const long long* __restrict__ tg,
-                                                        const float* __restrict__ inv_count, float* __restrict__ loss,
-                                                        int write_grad) {
-    pdl_wait();
-    __shared__ float red[8];
-    __shared__ float bc[2];
-    const int row = blockIdx.x, tid = threadIdx.x;
-    bf16* lr = logits + (size_t)row * ld;
-    const long long t = tg[row];
-    const float ic = *inv_count;
-    if (t == 0) {
-        if (write_grad)
-            for (int c = tid; c < ld; c += 256) lr[c] = __float2bfloat16(0.f);
-        return;
-    }
-    float m = -INFINITY;
-    for (int c = tid; c < C; c += 256) m = fmaxf(m, __bfloat162float(lr[c]));
-    m = warp_max(m);
-    if ((tid & 31) == 0) red[tid >> 5] = m;
-    __syncthreads();
-    if (tid == 0) {
-        float mm = red[0];
-        for (int w = 1; w < 8; ++w) mm = fmaxf(mm, red[w]);
-        bc[0] = mm;
-    }
-    __syncthreads();
-    m = bc[0];
-    float s = 0.f;
-    for (int c = tid; c < C; c += 256) s += __expf(__bfloat162float(lr[c]) - m);
-    s = warp_sum(s);
-    __syncthreads();
-    if ((tid & 31) == 0) red[tid >> 5] = s;
-    __syncthreads();
-    if (tid == 0) {
-        float ss = 0.f;
-        for (int w = 0; w < 8; ++w) ss += red[w];
-        bc[1] = ss;
-        float lse = m + logf(ss);
-        atomicAdd(loss, (lse - __bfloat162float(lr[t])) * ic);
-    }
-    __syncthreads();
-    if (!write_grad) return;
-    const float inv_s = 1.f / bc[1];
-    for (int c = tid; c < ld; c += 256) {
-        float gvl = 0.f;
-        if (c < C) {
-            gvl = __expf(__bfloat162float(lr[c]) - m) * inv_s;
-            if (c == (int)t) gvl -= 1.f;
-            gvl *= ic;
-        }
-        lr[c] = __float2bfloat16(gvl);
-    }
-}
-
-// Register-resident variant: the whole row (<= 256 x NCH x 8 logits) is read ONCE with 16-byte loads; exp(x - max) is
-// evaluated once per logit and kept in registers for the gradient pass; the row is written ONCE.
-// HBM traffic = 1 read + 1 write of the logits; ~10 instructions per logit.
-template <int NCH>
-__global__ void __launch_bounds__(256) ce_fwd_bwd_vec_kernel(bf16* __restrict__ logits, int ld, int C, const long long* __restrict__ tg,
-                                                            const float* __restrict__ inv_count, float* __restrict__ loss, int write_grad) {
-    pdl_wait();
-    __shared__ float red[8];
-    __shared__ float bc[3];
-    const int row = blockIdx.x, tid = threadIdx.x;
-    uint4* lr = reinterpret_cast<uint4*>(logits + (size_t)row * ld);
-    const int nchunks = ld >> 3;
-    const int t = (int)tg[row];
-    const float ic = *inv_count;
-    if (t == 0) {
-        if (write_grad)
-            for (int c = tid; c < nchunks; c += 256) lr[c] = make_uint4(0u, 0u, 0u, 0u);
-        return;
-    }
-    float e[NCH][8];
-    float m = -INFINITY;
-#pragma unroll
-    for (int i = 0; i < NCH; ++i) {
-        const int c = tid + i * 256;
-        if (c < nchunks) {
-            const uint4 q = lr[c];
-            const uint32_t u[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                float2 f = unpack_bf16(u[k]);
-                e[i][2 * k] = f.x;
-                e[i][2 * k + 1] = f.y;
-            }
-            if (c * 8 + 8 > C) {   // the single partial chunk: pad columns do not take part
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    if (c * 8 + k >= C) e[i][k] = -INFINITY;
-            }
-#pragma unroll
-            for (int k = 0; k < 8; ++k) m = fmaxf(m, e[i][k]);
-        }
-    }
-    m = warp_max(m);
-    if ((tid & 31) == 0) red[tid >> 5] = m;
-    __syncthreads();
-    if (tid == 0) {
-        float mm = red[0];
-        for (int w = 1; w < 8; ++w) mm = fmaxf(mm, red[w]);
-        bc[0] = mm;
-    }
-    __syncthreads();
-    m = bc[0];
-    const float ml2 = m * 1.4426950408889634f;
-    float ssum = 0.f;
-    // the thread that owns the target column remembers its logit
-    const int tc = t >> 3, ti = (tc - tid) >> 8;
-    float tlogit = 0.f;
-    const bool own = (tc >= tid) && (((tc - tid) & 255) == 0) && ti < NCH;
-#pragma unroll
-    for (int i = 0; i < NCH; ++i) {
-        const int c = tid + i * 256;
-        if (c < nchunks) {
-            if (own && i == ti) {
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    if (k == (t & 7)) tlogit = e[i][k];
-            }
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                e[i][k] = exp2f(fmaf(e[i][k], 1.4426950408889634f, -ml2));   // exp(x - m); exp2(-inf) = 0 for pad columns
-                ssum += e[i][k];
-            }
-        }
-    }
-    ssum = warp_sum(ssum);
-    __syncthreads();
-    if ((tid & 31) == 0) red[tid >> 5] = ssum;
-    __syncthreads();
-    if (tid == 0) {
-        float ss = 0.f;
-        for (int w = 0; w < 8; ++w) ss += red[w];
-        bc[1] = ss;
-    }
-    __syncthreads();
-    const float stot = bc[1];
-    if (own) atomicAdd(loss, (m + logf(stot) - tlogit) * ic);
-    if (!write_grad) return;
-    const float sc = ic / stot;
-#pragma unroll
-    for (int i = 0; i < NCH; ++i) {
-        const int c = tid + i * 256;
-        if (c < nchunks) {
-            float gk[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) gk[k] = e[i][k] * sc;
-            if (own && i == ti) {
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    if (k == (t & 7)) gk[k] -= ic;
-            }
-            lr[c] = make_uint4(pack_bf16(gk[0], gk[1]), pack_bf16(gk[2], gk[3]), pack_bf16(gk[4], gk[5]), pack_bf16(gk[6], gk[7]));
-        }
     }
 }
 

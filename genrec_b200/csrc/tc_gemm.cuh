@@ -548,20 +548,6 @@ GRB_DEVINL float exp_accurate(float x) {
     p = __fmaf_rn(p, r, 1.f);
     return p * __int_as_float(((int)n + 127) << 23);
 }
-// out = ACT(acc) -> fp32   (ACT 0: none, 1: silu) - the bias-free MLP layers of the RQ-VAE encoder (fp32-accurate split-bf16 GEMM)
-template <int ACT>
-struct TcEpiActF32 {
-    static constexpr int kOut = 3;
-    static constexpr bool kPre = false;
-    static constexpr bool kAux = false;
-    GRB_DEVINL void prepare() {}
-    GRB_DEVINL void operator()(int, int, float (&v)[32], float (&)[32], int) const {
-        if (ACT == 1) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = __fdiv_rn(v[i], 1.f + exp_accurate(-v[i]));
-        }
-    }
-};
 // out = ACT(res + acc + bias) + res2 -> fp32 : second pass of the split-bf16 GEMM (res = the sum of the five small cross terms;
 // bias [N] and res2 [M, ld] nullable: the linear layers and the residual connection of the fp32-exact HSTU block)
 template <int ACT>
@@ -603,14 +589,6 @@ struct TcEpiAtomicF32 {
         for (int i = 0; i < 32; ++i)
             if (i < nvalid) atomicAdd(dst + i, v[i] * scale);
     }
-};
-// plain bf16 store
-struct TcEpiBf16 {
-    static constexpr int kOut = 1;
-    static constexpr bool kPre = false;
-    static constexpr bool kAux = false;
-    GRB_DEVINL void prepare() {}
-    GRB_DEVINL void operator()(int, int, float (&)[32], float (&)[32], int) const {}
 };
 // plain fp32 store, arbitrary leading dimension
 struct TcEpiF32Plain {

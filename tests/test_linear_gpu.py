@@ -1,4 +1,4 @@
-"""GEMM building blocks through the C ABI (tcgen05/TMA path by default; GRB_GEMM=mma selects the mma.sync path) vs torch."""
+"""GEMM building blocks through the C ABI (tcgen05/TMA kernels) vs torch."""
 import pytest
 import torch
 
